@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the CMGAN hot path on B200 (contract in the task statement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--workload train_gd|gen_only]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--workload train_gd|gen_only] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], metric: utterances/sec, 2 s @ 16 kHz): per rank, one step = the reference's whole
@@ -14,12 +14,16 @@ Workload (BASELINE.json configs[2], metric: utterances/sec, 2 s @ 16 kHz): per r
 All of it is one CUDA graph per step.  Prints ONE JSON line on rank 0.
 """
 import argparse
+import io
 import json
 import os
 import subprocess
 import sys
 import threading
 import time
+
+# the benchmark leaves the tree it runs from untouched (it may be read-only): no __pycache__ for the modules it imports
+sys.dont_write_bytecode = True
 
 # stdout carries exactly one JSON line.  Libraries print there too (NCCL's version banner), so file descriptor 1 is pointed at
 # stderr for the whole run and the JSON line is written to the saved original descriptor by emit().
@@ -280,6 +284,10 @@ def run_ours(args):
     model = cmgan_b200.TSCNet(64, 201).to(dev).train()
     disc = cmgan_b200.Discriminator(16).to(dev).train() if gd else None
     trainer = FusedTrainer(model, disc)          # flat parameter/gradient buffers; rank-0 parameters win (train.py:68)
+    start_state = None
+    if args.dump_outputs:                        # the seeded state before any step: the dumped step starts from it
+        start_state = io.BytesIO()
+        trainer.save_checkpoint(start_state, full=True)
     clean, noisy = synth_batch(B, 1000 + rank, device=dev)
     hclean, hnoisy = synth_batch(B, 1000 + rank, pin=True)
     pesq_t = torch.full((B,), 0.5, device=dev)
@@ -350,6 +358,17 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     ms = timed(lambda: gstep(clean, noisy, pesq_t), args.steps)
+    if args.dump_outputs:
+        trained_state = io.BytesIO()
+        trainer.save_checkpoint(trained_state, full=True)
+        start_state.seek(0)
+        trainer.load_checkpoint(start_state)
+        gstep(clean, noisy, pesq_t)
+        barrier()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, trainer, gd)
+        trained_state.seek(0)
+        trainer.load_checkpoint(trained_state)
     losses = gstep(clean, noisy, pesq_t)
     loss_after = float(losses[0].item())
     dloss_after = float(losses[1].item()) if gd else None
@@ -404,6 +423,29 @@ def run_ours(args):
         torch.cuda.synchronize()
         sys.stderr.flush()
         os._exit(0)
+
+
+DUMP_AUDIO_BYTES = 32 << 20
+
+
+def dump_outputs(path, trainer, gd):
+    """write what one replay of the timed step computed from the seeded batch and the seeded start state, as float32 .npy files:
+    the losses, the enhanced waveforms (the first rows only, when the batch's exceed 32 MB) and the gradients.
+
+    The step starts from the state before any training step because the timed steps' weights carry every earlier step's rounding:
+    the gradient, statistics and loss reductions accumulate with float atomics in whatever order they land, and AdamW turns a
+    rounding-level gradient (conv biases in front of an InstanceNorm, mathematically zero) into a +-lr move.  For the same reason
+    the updated parameters are not written: the gradients are what the step computed from them."""
+    import numpy as np
+    audio = trainer.last["est_audio"]
+    arrays = {"generator_loss": trainer.static_losses[0] if gd else trainer.static_loss,
+              "est_audio": audio[:max(1, DUMP_AUDIO_BYTES // (audio.shape[1] * audio.element_size()))],
+              "generator_grads": trainer.gg}
+    if gd:
+        arrays.update(discriminator_loss=trainer.static_losses[1], discriminator_grads=trainer.gd)
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def extras(args, out, trainer, model, dev, step_ms):
@@ -641,7 +683,12 @@ def main():
     ap.add_argument("--no-gpu-eager", action="store_true", help="skip the GPU-eager reference leg")
     ap.add_argument("--no-extras", action="store_true", help="headline only (no forward-only / roofline / baseline legs)")
     ap.add_argument("--precision", default="tf32", choices=["tf32", "fp32"], help="dense contractions: tcgen05 tf32 (default) or exact fp32 FFMA")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, replay the timed step once from the seeded start state and write what it computed to "
+                         "DIR/<name>.npy (float32; the same inputs every run, so two builds compare output for output)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

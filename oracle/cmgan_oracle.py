@@ -11,10 +11,10 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s CPU-baseline /
 ``--impl reference`` legs may import it, and only as the *checker* (or the thing
 timed as the CPU baseline); the product package ``cmgan_b200`` never imports it.
 
-Parity status: **pinned**.  ``tests/test_oracle_vs_reference.py`` imports the
-reference's own modules from ``/root/reference/src`` (when that tree exists, i.e.
-in the build container) and checks every function below against them on the
-shipped checkpoint; ``tools/make_golden.py`` (committed) wrote the fixtures under
+Parity status: **pinned**.  ``tests/test_oracle_vs_reference.py`` checks the
+generator, the power compression and the train-mode discriminator against outputs
+the reference's own modules computed on the shipped checkpoint
+(``tools/make_golden_oracle_pins.py``); ``tools/make_golden.py`` (committed) wrote the fixtures under
 ``tests/golden/`` from the *reference* modules, and ``tests/test_oracle_golden.py``
 checks this oracle against those fixtures everywhere (GPU box included, where
 ``/root/reference`` does not exist).  The one unpinned quantity is PESQ (the ``pesq``
