@@ -63,12 +63,17 @@ class _Sums:
         return (self.buf, o)
 
 
-def _inst_norm_site(x, ldx, G, rows, Cn, gamma, beta, tabs: _Tabs, c0, slope_w, sums: _Sums):
-    """InstanceNorm2d statistics (ref: generator.py:35) -> tables at channel offset c0 of ``tabs``"""
+def _inst_norm_site(x, ldx, G, rows, Cn, gamma, beta, tabs: _Tabs, c0, slope_w, sums: _Sums, frames=None, T=None):
+    """InstanceNorm2d statistics (ref: generator.py:35) -> tables at channel offset c0 of ``tabs``.
+    ``frames`` (ragged batch, device int32 (G,)): group g spans its first frames[g] of T frames (rows / T rows each)"""
     s = sums.take(G * Cn * 2)
-    call("cmgan_norm_stats", x, ldx, G, rows, Cn, s)
-    call("cmgan_norm_finalize", s, rows, G, Cn, 0, gamma, beta, None, None, 0.0, (tabs.scale, c0), (tabs.shift, c0), (tabs.mean, c0),
-         (tabs.rstd, c0), tabs.width)
+    tabs_out = ((tabs.scale, c0), (tabs.shift, c0), (tabs.mean, c0), (tabs.rstd, c0), tabs.width)
+    if frames is not None:
+        call("cmgan_norm_stats_varlen", x, ldx, G, rows, Cn, frames, rows // T, s)
+        call("cmgan_norm_finalize_varlen", s, frames, rows // T, T, G, Cn, gamma, beta, *tabs_out)
+    else:
+        call("cmgan_norm_stats", x, ldx, G, rows, Cn, s)
+        call("cmgan_norm_finalize", s, rows, G, Cn, 0, gamma, beta, None, None, 0.0, *tabs_out)
     if slope_w is not None:
         call("cmgan_copy_rows", slope_w, Cn, (tabs.slope, c0), Cn, 1, Cn)
 
@@ -93,9 +98,13 @@ def _rnd() -> int:
 
 
 # ====================================================================================== conformer block
-def conformer_fwd(x, P, p, B, T, F2, axis, training, seed, block_id, sums: _Sums, save: Optional[dict]):
+def conformer_fwd(x, P, p, B, T, F2, axis, training, seed, block_id, sums: _Sums, save: Optional[dict], frames=None):
     """ConformerBlock + the outer TSCB residual (ref: conformer.py:216-222, generator.py:95,97).
-    x: (M, 64) rows of the (B, T, F2) grid; axis 0 = sequences along T, 1 = along F2.  Returns LN(x4) + x."""
+    x: (M, 64) rows of the (B, T, F2) grid; axis 0 = sequences along T, 1 = along F2.  Returns LN(x4) + x.
+    ``frames`` (inference only, device int32 (B,)): ragged batch -- item b has frames[b] valid frames; attention and the depthwise
+    convolution never read the rows of padded frames, every other operation works row by row."""
+    if frames is not None and (training or save is not None):
+        raise ValueError("conformer_fwd: ragged batches (frames) are inference only")
     dev = x.device
     M = x.shape[0]
     dp = FF_DROP if training else 0.0
@@ -144,8 +153,14 @@ def conformer_fwd(x, P, p, B, T, F2, axis, training, seed, block_id, sums: _Sums
         gemm(A=xn2, lda=C, W=Wkv, sb_k=1, sb_n=C, C=(qkv, C), ldc=3 * C, M=M, N=2 * C, Cin=C)
     ctx = _empty(M, C, dev=dev)
     lse = _empty(M, 4, dev=dev)
-    call(("cmgan_attention_fwd_tc" if ops.ATTN_TC else "cmgan_attention_fwd_tf32") if ops.PRECISION == 1 else "cmgan_attention_fwd", qkv, P[f"{p}.attn.fn.rel_pos_emb.weight"], B, T, F2, axis,
-         ctx, lse)
+    if frames is not None:
+        if ops.PRECISION == 1 and ops.ATTN_TC:
+            raise ValueError("the tcgen05 attention forward (CMGAN_ATTN_TC=1) has no ragged-batch variant; unset it to pass frames")
+        call("cmgan_attention_fwd_tf32_varlen" if ops.PRECISION == 1 else "cmgan_attention_fwd_varlen", qkv, P[f"{p}.attn.fn.rel_pos_emb.weight"],
+             B, T, F2, axis, frames, ctx, lse)
+    else:
+        call(("cmgan_attention_fwd_tc" if ops.ATTN_TC else "cmgan_attention_fwd_tf32") if ops.PRECISION == 1 else "cmgan_attention_fwd", qkv, P[f"{p}.attn.fn.rel_pos_emb.weight"], B, T, F2, axis,
+             ctx, lse)
     x2 = _empty(M, C, dev=dev)
     gemm(A=ctx, lda=C, W=P[f"{p}.attn.fn.to_out.weight"], sb_k=1, sb_n=C, bias=P[f"{p}.attn.fn.to_out.bias"], C=x2, ldc=C, M=M, N=C, Cin=C,
          epi=EPI_DROP_RES, alpha=1.0, R=x1, ldr=C, seed=sd[2], drop_p=da)
@@ -156,7 +171,10 @@ def conformer_fwd(x, P, p, B, T, F2, axis, training, seed, block_id, sums: _Sums
     d = _empty(M, 2 * C, dev=dev)
     # training: the BatchNorm batch statistics (sum, sum of squares per channel) come out of the depthwise kernel's epilogue
     s = sums.take(2 * C * 2) if training else None
-    call("cmgan_glu_dwconv_fwd", g, P[f"{p}.conv.net.4.conv.weight"], P[f"{p}.conv.net.4.conv.bias"], B, T, F2, axis, d, s)
+    if frames is not None:
+        call("cmgan_glu_dwconv_fwd_varlen", g, P[f"{p}.conv.net.4.conv.weight"], P[f"{p}.conv.net.4.conv.bias"], B, T, F2, axis, frames, d)
+    else:
+        call("cmgan_glu_dwconv_fwd", g, P[f"{p}.conv.net.4.conv.weight"], P[f"{p}.conv.net.4.conv.bias"], B, T, F2, axis, d, s)
     bn = _Tabs(1, 2 * C, dev)
     bnp = (P[f"{p}.conv.net.5.weight"], P[f"{p}.conv.net.5.bias"], P[f"{p}.conv.net.5.running_mean"], P[f"{p}.conv.net.5.running_var"])
     if training:

@@ -66,13 +66,19 @@ __device__ __forceinline__ void stage_E(float* dst, const float* E, int rfirst, 
 }
 
 // ------------------------------------------------------------------------------------------ forward
+// VAR: ragged batch (frames, axis; common.cuh): a sequence's length is its own (time axis) and sequences of padded frames do no work
+// (frequency axis), so a valid row is computed with exactly the arithmetic of a run on its utterance alone.
+template <bool VAR>
 __global__ void __launch_bounds__(NTH) attn_fwd_kernel(const float* __restrict__ qkv, SeqGeom g, const float* __restrict__ E,
-                                                       float* __restrict__ ctx, float* __restrict__ lse) {
+                                                       float* __restrict__ ctx, float* __restrict__ lse, const int* __restrict__ frames,
+                                                       int axis) {
     __shared__ __align__(16) float Ks[TILE * D], Vs[TILE * D], Es[WROWS * WLD];
     const int s = blockIdx.x / H, h = blockIdx.x % H;
     const int i0 = blockIdx.y * NTH, il = threadIdx.x, i = i0 + il;
+    const int L = VAR ? varlen_seq_len(g, frames, axis, s) : g.L;
+    if (VAR && i0 >= L) return;
     const long base = seq_base(g, s);
-    const bool active = i < g.L;
+    const bool active = i < L;
     float q[D], acc[D];
 #pragma unroll
     for (int d = 0; d < D; ++d) { q[d] = 0.f; acc[d] = 0.f; }
@@ -82,11 +88,11 @@ __global__ void __launch_bounds__(NTH) attn_fwd_kernel(const float* __restrict__
         for (int d = 0; d < D; ++d) q[d] *= SCALE_LOG2E;
     }
     float mrun = -INFINITY, lrun = 0.f;
-    for (int j0 = 0; j0 < g.L; j0 += TILE) {
-        const int nk = min(TILE, g.L - j0);
+    for (int j0 = 0; j0 < L; j0 += TILE) {
+        const int nk = min(TILE, L - j0);
         __syncthreads();
-        stage_rows16(Ks, qkv + CQ + h * D, base, g.tok_stride, j0, nk, g.L, 1.f);
-        stage_rows16(Vs, qkv + 2 * CQ + h * D, base, g.tok_stride, j0, nk, g.L, 1.f);
+        stage_rows16(Ks, qkv + CQ + h * D, base, g.tok_stride, j0, nk, L, 1.f);
+        stage_rows16(Vs, qkv + 2 * CQ + h * D, base, g.tok_stride, j0, nk, L, 1.f);
         // r = i - j = (i0 - j0) + (il - jl);  window row w = il - jl + TILE - 1
         stage_E(Es, E, i0 - j0 - (TILE - 1), NTH + nk - 1 + (TILE - nk));
         __syncthreads();
@@ -354,14 +360,27 @@ static SeqGeom geom_from(int B, int T, int F, int axis) { return make_seq_geom(B
 
 // qkv (B*T*F, 192) -> ctx (B*T*F, 64), lse (B*T*F, 4) (base-2 log-sum-exp of the scaled logits; may be null).
 // axis 0: sequences along T (time conformer, generator.py:94); axis 1: along F (freq conformer, generator.py:96).
-CMGAN_API int cmgan_attention_fwd(const float* qkv, const float* E, int B, int T, int F, int axis, float* ctx, float* lse, void* stream) {
+// frames (optional, device int[B]): ragged batch; rows of padded frames are neither read nor written.
+static int attention_fwd_launch(const float* qkv, const float* E, int B, int T, int F, int axis, const int* frames, float* ctx, float* lse,
+                                void* stream) {
     CMGAN_REQUIRE(qkv && E && ctx, "cmgan_attention_fwd: null pointer");
     CMGAN_REQUIRE(axis == 0 || axis == 1, "cmgan_attention_fwd: axis must be 0 (time) or 1 (freq)");
     SeqGeom g = geom_from(B, T, F, axis);
     if (g.n_seq == 0 || g.L == 0) return 0;
     dim3 grid(g.n_seq * H, cdiv(g.L, NTH));
-    attn_fwd_kernel<<<grid, NTH, 0, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse);
+    if (frames) attn_fwd_kernel<true><<<grid, NTH, 0, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse, frames, axis);
+    else attn_fwd_kernel<false><<<grid, NTH, 0, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse, nullptr, axis);
     return cmgan_check_launch("attn_fwd_kernel");
+}
+
+CMGAN_API int cmgan_attention_fwd(const float* qkv, const float* E, int B, int T, int F, int axis, float* ctx, float* lse, void* stream) {
+    return attention_fwd_launch(qkv, E, B, T, F, axis, nullptr, ctx, lse, stream);
+}
+
+CMGAN_API int cmgan_attention_fwd_varlen(const float* qkv, const float* E, int B, int T, int F, int axis, const int* frames, float* ctx, float* lse,
+                                         void* stream) {
+    CMGAN_REQUIRE(frames, "cmgan_attention_fwd_varlen: null frames");
+    return attention_fwd_launch(qkv, E, B, T, F, axis, frames, ctx, lse, stream);
 }
 
 // dqkv (B*T*F, 192) fully overwritten; dE (1025, 16) accumulated (+=); delta (B*T*F, 4) scratch.

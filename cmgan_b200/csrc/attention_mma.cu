@@ -81,17 +81,22 @@ __device__ __forceinline__ void stage_tile_async(float* buf, const float* __rest
 // NBUF = 2: the next key tile is staged while the current one is processed (62.5 KB of shared memory, 3 blocks / SM).
 // NBUF = 1: one tile buffer, staged and waited for at the top of each iteration (42 KB, 5 blocks / SM): the load latency is hidden by the
 // other resident blocks instead of by a second buffer.
-template <int NBUF>
+// VAR: ragged batch (frames, axis; common.cuh): the key and query length of a sequence is its own (time axis), sequences of padded
+// frames do no work (frequency axis); a valid row gets exactly the arithmetic of a run on its utterance alone.
+template <int NBUF, bool VAR>
 __global__ void __launch_bounds__(128) attn_fwd_mma_kernel(const float* __restrict__ qkv, SeqGeom g, const float* __restrict__ E,
-                                                           float* __restrict__ ctx, float* __restrict__ lse) {
+                                                           float* __restrict__ ctx, float* __restrict__ lse, const int* __restrict__ frames,
+                                                           int axis) {
     extern __shared__ __align__(16) float smem_fwd[];          // tile buffers [NBUF][TILE_FLOATS] | Rs[4][16 * LDR]
     float* Rs0 = smem_fwd + NBUF * TILE_FLOATS;
     const int s = blockIdx.x / H, h = blockIdx.x % H;
     const int i0 = blockIdx.y * QB;
+    const int L = VAR ? varlen_seq_len(g, frames, axis, s) : g.L;
+    if (VAR && i0 >= L) return;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, gq = lane >> 2, t = lane & 3;
     const long base = seq_base(g, s);
     const int iw = i0 + warp * 16;                    // first query of this warp
-    const bool warp_active = iw < g.L;
+    const bool warp_active = iw < L;
 
     // ---- Q fragments (rows gq, gq+8), scaled and rounded once
     float qa[2][4];
@@ -101,7 +106,7 @@ __global__ void __launch_bounds__(128) attn_fwd_mma_kernel(const float* __restri
         for (int r = 0; r < 4; ++r) {
             const int row = iw + gq + (r & 1) * 8, col = t + (r >> 1) * 4 + ks * 8;
             float v = 0.f;
-            if (row < g.L) v = __ldg(qkv + (base + (long)row * g.tok_stride) * LDQ + h * D + col) * SCALE_LOG2E;
+            if (row < L) v = __ldg(qkv + (base + (long)row * g.tok_stride) * LDQ + h * D + col) * SCALE_LOG2E;
             qa[ks][r] = tf32r(v);
         }
     float o[2][4];
@@ -115,23 +120,23 @@ __global__ void __launch_bounds__(128) attn_fwd_mma_kernel(const float* __restri
     const float* vsrc = qkv + h * D + 2 * CQ;
     // window row w <-> relative distance r = (i0 - j0 - (KT - 1)) + w
     if (NBUF == 2) {
-        stage_tile_async(smem_fwd, ksrc, LDQ, vsrc, LDQ, base, g.tok_stride, 0, g.L, E, i0 - (KT - 1), tid);
+        stage_tile_async(smem_fwd, ksrc, LDQ, vsrc, LDQ, base, g.tok_stride, 0, L, E, i0 - (KT - 1), tid);
         cp_async_commit();
     }
-    for (int j0 = 0, it = 0; j0 < g.L; j0 += KT, ++it) {
-        const int nk = min(KT, g.L - j0);
+    for (int j0 = 0, it = 0; j0 < L; j0 += KT, ++it) {
+        const int nk = min(KT, L - j0);
         const float* Ks = smem_fwd + (NBUF == 2 ? (it & 1) : 0) * TILE_FLOATS;
         const float* Vs = Ks + KT * LDS_;
         const float* Es = Vs + KT * LDS_;
         __syncthreads();                              // every warp is done with the buffer the next tile is staged into
         if (NBUF == 2) {
-            if (j0 + KT < g.L)
-                stage_tile_async(smem_fwd + ((it + 1) & 1) * TILE_FLOATS, ksrc, LDQ, vsrc, LDQ, base, g.tok_stride, j0 + KT, g.L, E,
+            if (j0 + KT < L)
+                stage_tile_async(smem_fwd + ((it + 1) & 1) * TILE_FLOATS, ksrc, LDQ, vsrc, LDQ, base, g.tok_stride, j0 + KT, L, E,
                                  i0 - (j0 + KT) - (KT - 1), tid);
             cp_async_commit();
             cp_async_wait<1>();                       // this tile has landed (the group just committed may still be in flight)
         } else {
-            stage_tile_async(smem_fwd, ksrc, LDQ, vsrc, LDQ, base, g.tok_stride, j0, g.L, E, i0 - j0 - (KT - 1), tid);
+            stage_tile_async(smem_fwd, ksrc, LDQ, vsrc, LDQ, base, g.tok_stride, j0, L, E, i0 - j0 - (KT - 1), tid);
             cp_async_commit();
             cp_async_wait<0>();
         }
@@ -235,7 +240,7 @@ __global__ void __launch_bounds__(128) attn_fwd_mma_kernel(const float* __restri
 #pragma unroll
     for (int hrow = 0; hrow < 2; ++hrow) {
         const int i = iw + gq + hrow * 8;
-        if (i >= g.L) continue;
+        if (i >= L) continue;
         const float inv = 1.f / lrun[hrow];
         const long row = base + (long)i * g.tok_stride;
 #pragma unroll
@@ -702,12 +707,25 @@ CMGAN_API int cmgan_attention_fwd_tf32_nbuf(const float* qkv, const float* E, in
     const int smem = (nbuf * TILE_FLOATS + 4 * 16 * LDR) * (int)sizeof(float);
     static bool attr_set = false;
     if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(attn_fwd_mma_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (2 * TILE_FLOATS + 4 * 16 * LDR) * (int)sizeof(float));
+        cudaError_t e = cudaFuncSetAttribute(attn_fwd_mma_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (2 * TILE_FLOATS + 4 * 16 * LDR) * (int)sizeof(float));
         CMGAN_REQUIRE(e == cudaSuccess, "cmgan_attention_fwd_tf32: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
         attr_set = true;
     }
-    if (nbuf == 2) attn_fwd_mma_kernel<2><<<grid, 128, smem, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse);
-    else attn_fwd_mma_kernel<1><<<grid, 128, smem, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse);
+    if (nbuf == 2) attn_fwd_mma_kernel<2, false><<<grid, 128, smem, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse, nullptr, axis);
+    else attn_fwd_mma_kernel<1, false><<<grid, 128, smem, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse, nullptr, axis);
+    return cmgan_check_launch("attn_fwd_mma_kernel");
+}
+
+// ragged batch (frames: device int[B], 1 <= frames[b] <= T): rows of padded frames are neither read nor written
+CMGAN_API int cmgan_attention_fwd_tf32_varlen(const float* qkv, const float* E, int B, int T, int F, int axis, const int* frames, float* ctx,
+                                              float* lse, void* stream) {
+    CMGAN_REQUIRE(qkv && E && ctx && frames, "cmgan_attention_fwd_tf32_varlen: null pointer");
+    CMGAN_REQUIRE(axis == 0 || axis == 1, "cmgan_attention_fwd_tf32_varlen: axis must be 0 (time) or 1 (freq)");
+    SeqGeom g = make_seq_geom(B, T, F, axis);
+    if (g.n_seq == 0 || g.L == 0) return 0;
+    dim3 grid(g.n_seq * H, cdiv(g.L, QB));
+    const int smem = (FWD_NBUF_DEFAULT * TILE_FLOATS + 4 * 16 * LDR) * (int)sizeof(float);
+    attn_fwd_mma_kernel<FWD_NBUF_DEFAULT, true><<<grid, 128, smem, (cudaStream_t)stream>>>(qkv, g, E, ctx, lse, frames, axis);
     return cmgan_check_launch("attn_fwd_mma_kernel");
 }
 

@@ -118,3 +118,19 @@ static inline SeqGeom make_seq_geom(int B, int T, int F, int axis /*0 = time, 1 
     else           { g.n_seq = B * T; g.L = F; g.n_inner = T; g.outer_stride = (long)T * F; g.inner_stride = F; g.tok_stride = 1; }
     return g;
 }
+
+// ---- ragged batches (inference) ------------------------------------------------------------------------
+// A ragged batch is the (B, T, F) grid padded along time: batch item b holds frames[b] valid frames, the rows t >= frames[b] are
+// padding and may hold anything (NaN included).  Kernels that combine rows along time never read a padded row.
+// Frame count of item b, clamped to [0, T] so that a bad length cannot move a load outside the tensor.
+__device__ __forceinline__ int varlen_frames(const int* __restrict__ frames, int b, int T) {
+    const int n = __ldg(frames + b);
+    return n < 0 ? 0 : (n > T ? T : n);
+}
+// Tokens of sequence s on a ragged grid: time axis (axis 0) -> frames[b] of its batch item; frequency axis -> all of them for a valid
+// frame, none for a padded one.  (s / n_inner is the batch item on both axes.)
+__device__ __forceinline__ int varlen_seq_len(const SeqGeom& g, const int* __restrict__ frames, int axis, int s) {
+    const int b = s / g.n_inner;
+    if (axis == 0) return varlen_frames(frames, b, g.L);
+    return (s % g.n_inner) < varlen_frames(frames, b, g.n_inner) ? g.L : 0;
+}

@@ -58,11 +58,35 @@ __device__ __forceinline__ void store_chunk(const ChunkRegs& r, float* U, float*
     }
 }
 
+// Ragged batch (common.cuh): the (sequence, tile) space holds the valid sequences only, each with its own tile count -- batch item b
+// contributes nseq_b sequences of tps_b tiles (time axis: F sequences of frames[b] tokens; frequency axis: frames[b] sequences of F
+// tokens).  A flat tile index is mapped back by a walk over the batch items (B is small; one walk per contiguous run of a block).
+__device__ __forceinline__ long varlen_items(const SeqGeom& sg, const int* __restrict__ frames, int axis, int b, int& L, int& tps) {
+    const int n = varlen_frames(frames, b, axis == 0 ? sg.L : sg.n_inner);
+    L = axis == 0 ? n : sg.L;
+    tps = (L + CK - 1) / CK;
+    return (long)(axis == 0 ? sg.n_inner : n) * tps;
+}
+__device__ long varlen_total(const SeqGeom& sg, const int* __restrict__ frames, int axis) {
+    long total = 0;
+    int L, tps;
+    for (int b = 0; b < sg.n_seq / sg.n_inner; ++b) total += varlen_items(sg, frames, axis, b, L, tps);
+    return total;
+}
+// flat tile index (< varlen_total) -> sequence s, tile k within it, tiles / tokens of that sequence
+__device__ __forceinline__ void varlen_tile(const SeqGeom& sg, const int* __restrict__ frames, int axis, long tile, int& s, int& k, int& tps, int& L) {
+    int b = 0;
+    for (long cnt; tile >= (cnt = varlen_items(sg, frames, axis, b, L, tps)); ++b) tile -= cnt;
+    s = b * sg.n_inner + (int)(tile / tps);
+    k = (int)(tile % tps);
+}
+
 // forward.  bn_sums (optional): per-channel sum / sum of squares of the output (sums[c * 2 + {0, 1}], BatchNorm1d batch statistics,
-// conformer.py:169) accumulated here instead of by a separate pass over `out`.
+// conformer.py:169) accumulated here instead of by a separate pass over `out`.  VAR: ragged batch (frames, axis), see varlen_tile.
+template <bool VAR>
 __global__ void __launch_bounds__(256, 3) glu_dwconv_fwd_kernel(const float* __restrict__ g, SeqGeom sg, const float* __restrict__ w,
                                                                 const float* __restrict__ bias, float* __restrict__ out,
-                                                                double* __restrict__ bn_sums) {
+                                                                double* __restrict__ bn_sums, const int* __restrict__ frames, int axis) {
     __shared__ __align__(16) float U[RING * CH];
     const int c = threadIdx.x & (CH - 1), half = threadIdx.x >> 7;
     float wr[KS];
@@ -70,25 +94,30 @@ __global__ void __launch_bounds__(256, 3) glu_dwconv_fwd_kernel(const float* __r
     for (int k = 0; k < KS; ++k) wr[k] = __ldg(w + c * KS + k);
     const float bs = __ldg(bias + c);
     float s1 = 0.f, s2 = 0.f;
-    const int tps = (sg.L + CK - 1) / CK;
-    const long total = (long)sg.n_seq * tps;
+    const int tps_u = (sg.L + CK - 1) / CK;
+    const long total = VAR ? varlen_total(sg, frames, axis) : (long)sg.n_seq * tps_u;
     long tile = total * blockIdx.x / gridDim.x;
     const long hi = total * (blockIdx.x + 1) / gridDim.x;
     ChunkRegs regs;
     while (tile < hi) {
-        const int s = (int)(tile / tps), k0 = (int)(tile % tps);
+        int s, k0, tps = tps_u, L = sg.L;
+        if (VAR) {
+            varlen_tile(sg, frames, axis, tile, s, k0, tps, L);
+        } else {
+            s = (int)(tile / tps); k0 = (int)(tile % tps);
+        }
         const int kend = (int)min((long)tps, k0 + (hi - tile));
         const long base = seq_base(sg, s);
         __syncthreads();                                        // the previous run is done with the ring
 #pragma unroll 1
         for (int ch = k0 - 1; ch <= k0 + 1; ++ch) {
-            load_chunk<false>(regs, g, nullptr, base, sg.tok_stride, ch, sg.L);
+            load_chunk<false>(regs, g, nullptr, base, sg.tok_stride, ch, L);
             store_chunk<false>(regs, U, nullptr, nullptr, ch);
         }
         __syncthreads();
 #pragma unroll 1
         for (int k = k0; k < kend; ++k) {
-            load_chunk<false>(regs, g, nullptr, base, sg.tok_stride, k + 2, sg.L);
+            load_chunk<false>(regs, g, nullptr, base, sg.tok_stride, k + 2, L);
             const int tok0 = k * CK + half * TOK;
             const int rs = (tok0 - PADL) & (RING - 1), wm = RING - rs;          // sweep row m lives at ring row (rs + m) mod 64
             const float* p1 = U + rs * CH + c;
@@ -106,7 +135,7 @@ __global__ void __launch_bounds__(256, 3) glu_dwconv_fwd_kernel(const float* __r
 #pragma unroll
             for (int i = 0; i < TOK; ++i) {
                 const int tok = tok0 + i;
-                if (tok < sg.L) {
+                if (tok < L) {
                     out[(base + (long)tok * sg.tok_stride) * CH + c] = acc[i];
                     s1 += acc[i];
                     s2 = fmaf(acc[i], acc[i], s2);
@@ -225,15 +254,29 @@ int resident_grid(long total, int per_sm) {
 
 }  // namespace
 
-CMGAN_API int cmgan_glu_dwconv_fwd(const float* g, const float* w, const float* bias, int B, int T, int F, int axis, float* out,
-                                   double* bn_sums, void* stream) {
+static int glu_dwconv_fwd_launch(const float* g, const float* w, const float* bias, int B, int T, int F, int axis, const int* frames, float* out,
+                                 double* bn_sums, void* stream) {
     CMGAN_REQUIRE(g && w && bias && out && (((uintptr_t)g) & 15) == 0, "cmgan_glu_dwconv_fwd: bad pointer");
     CMGAN_REQUIRE(axis == 0 || axis == 1, "cmgan_glu_dwconv_fwd: bad axis");
     SeqGeom sg = make_seq_geom(B, T, F, axis);
     if (sg.n_seq == 0 || sg.L == 0) return 0;
-    const long total = (long)sg.n_seq * cdiv(sg.L, CK);
-    glu_dwconv_fwd_kernel<<<resident_grid(total, 3), 256, 0, (cudaStream_t)stream>>>(g, sg, w, bias, out, bn_sums);
+    const long total = (long)sg.n_seq * cdiv(sg.L, CK);      // a ragged batch has at most this many tiles
+    if (frames) glu_dwconv_fwd_kernel<true><<<resident_grid(total, 3), 256, 0, (cudaStream_t)stream>>>(g, sg, w, bias, out, nullptr, frames, axis);
+    else glu_dwconv_fwd_kernel<false><<<resident_grid(total, 3), 256, 0, (cudaStream_t)stream>>>(g, sg, w, bias, out, bn_sums, nullptr, axis);
     return cmgan_check_launch("glu_dwconv_fwd_kernel");
+}
+
+CMGAN_API int cmgan_glu_dwconv_fwd(const float* g, const float* w, const float* bias, int B, int T, int F, int axis, float* out,
+                                   double* bn_sums, void* stream) {
+    return glu_dwconv_fwd_launch(g, w, bias, B, T, F, axis, nullptr, out, bn_sums, stream);
+}
+
+// ragged batch (frames: device int[B], 1 <= frames[b] <= T); inference only (no BatchNorm batch statistics).  Rows of padded frames are
+// neither read nor written, and the persistent partition spans the valid tiles only.
+CMGAN_API int cmgan_glu_dwconv_fwd_varlen(const float* g, const float* w, const float* bias, int B, int T, int F, int axis, const int* frames,
+                                          float* out, void* stream) {
+    CMGAN_REQUIRE(frames, "cmgan_glu_dwconv_fwd_varlen: null frames");
+    return glu_dwconv_fwd_launch(g, w, bias, B, T, F, axis, frames, out, nullptr, stream);
 }
 
 CMGAN_API int cmgan_glu_dwconv_bwd(const float* g, const float* dz, const float* w, int B, int T, int F, int axis, float* dg, float* dw,

@@ -11,9 +11,11 @@ namespace {
 constexpr int NFFT = 400, HOP = 100, NF = 201;
 
 // ------------------------------------------------------------------ RMS scale: c[b] = sqrt(L / sum x^2)
-__global__ void rms_scale_kernel(const float* __restrict__ x, long ldx, int L, float* __restrict__ c) {
+// lens (optional, ragged batch): row b holds lens[b] <= L samples
+__global__ void rms_scale_kernel(const float* __restrict__ x, long ldx, int L, float* __restrict__ c, const int* __restrict__ lens) {
     __shared__ double sm[32];
     const float* p = x + (long)blockIdx.x * ldx;
+    if (lens) L = min(__ldg(lens + blockIdx.x), L);
     double s = 0.0;
     for (int i = threadIdx.x; i < L; i += blockDim.x) { float v = __ldg(p + i); s += (double)v * v; }
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
@@ -37,6 +39,27 @@ __global__ void pad_reflect_kernel(const float* __restrict__ x, long ldx, int L,
         if (j < 0) j = -j;
         if (j >= L) j = 2 * (L - 1) - j;
         v = __ldg(x + (long)b * ldx + j) * (c ? c[b] : 1.f);
+    }
+    xp[(long)b * Lp + i] = v;
+}
+
+// ragged batch of clips, one kernel for what evaluation.py:25-29 + train.py:77-87 do to one file: row b (lens[b] > 200 samples) is
+// wrap-padded with its own head to Lw = ceil(lens[b] / 100) * 100 samples, reflect-padded by 200 on both sides and scaled by c[b]:
+//   xp[b, i] = c[b] * u[reflect(i - 200)], i < Lw + 400,   u[j] = x[b, j < lens[b] ? j : j - lens[b]];   zero from Lw + 400 up to Lp
+__global__ void wrap_pad_reflect_kernel(const float* __restrict__ x, long ldx, const int* __restrict__ lens, const float* __restrict__ c,
+                                        float* __restrict__ xp, int Lp) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = blockIdx.y;
+    if (i >= Lp) return;
+    const int L = __ldg(lens + b);
+    const int Lw = (L + HOP - 1) / HOP * HOP;
+    float v = 0.f;
+    if (i < Lw + NFFT) {
+        int j = i - NFFT / 2;
+        if (j < 0) j = -j;
+        if (j >= Lw) j = 2 * (Lw - 1) - j;
+        if (j >= L) j -= L;
+        v = __ldg(x + (long)b * ldx + j) * c[b];
     }
     xp[(long)b * Lp + i] = v;
 }
@@ -144,6 +167,34 @@ __global__ void ola_kernel(const float* __restrict__ frames, int T, const float*
     }
     s *= inv_env[n];
     if (c_div) s /= c_div[b];
+    y[(long)b * ldy + n] = s;
+}
+
+// overlap-add of a ragged batch: utterance b has nframes[b] <= T frames.  The window-square envelope of each utterance is summed here in
+// float64, frame by frame in increasing t exactly like signal._inv_envelope (win_sq = the float64 squared window), so every sample
+// equals that of the per-utterance ola_kernel.  Samples from 100 (nframes[b] - 1) on are zero.
+__global__ void ola_varlen_kernel(const float* __restrict__ frames, int T, const int* __restrict__ nframes, const double* __restrict__ win_sq,
+                                  const float* __restrict__ c_div, float* __restrict__ y, long ldy) {
+    const int n = blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = blockIdx.y;
+    if (n >= HOP * (T - 1)) return;
+    const int Tb = min(__ldg(nframes + b), T);
+    float s = 0.f;
+    if (n < HOP * (Tb - 1)) {
+        const int p = n + NFFT / 2;
+        int t_hi = p / HOP; if (t_hi > Tb - 1) t_hi = Tb - 1;
+        int t_lo = (p - NFFT + HOP) / HOP; if (p - NFFT + 1 <= 0) t_lo = 0;
+        double env = 0.0;
+        for (int t = t_lo; t <= t_hi; ++t) {
+            int k = p - t * HOP;
+            if (k >= 0 && k < NFFT) {
+                s += __ldg(frames + ((long)b * T + t) * NFFT + k);
+                env += __ldg(win_sq + k);
+            }
+        }
+        s *= (float)(1.0 / env);
+        if (c_div) s /= c_div[b];
+    }
     y[(long)b * ldy + n] = s;
 }
 
@@ -360,8 +411,26 @@ __global__ void recombine_bwd_kernel(const float* __restrict__ m1, MaskTail mt, 
 CMGAN_API int cmgan_rms_scale(const float* x, long long ldx, int B, int L, float* c, void* stream) {
     CMGAN_REQUIRE(x && c && L > 0, "cmgan_rms_scale: bad arguments");
     if (B == 0) return 0;
-    rms_scale_kernel<<<B, 256, 0, (cudaStream_t)stream>>>(x, ldx, L, c);
+    rms_scale_kernel<<<B, 256, 0, (cudaStream_t)stream>>>(x, ldx, L, c, nullptr);
     return cmgan_check_launch("rms_scale_kernel");
+}
+
+// ragged batch: c[b] = sqrt(lens[b] / sum of the first lens[b] samples of row b squared); ldx >= every lens[b]
+CMGAN_API int cmgan_rms_scale_varlen(const float* x, long long ldx, int B, const int* lens, float* c, void* stream) {
+    CMGAN_REQUIRE(x && lens && c && ldx > 0, "cmgan_rms_scale_varlen: bad arguments");
+    if (B == 0) return 0;
+    rms_scale_kernel<<<B, 256, 0, (cudaStream_t)stream>>>(x, ldx, (int)ldx, c, lens);
+    return cmgan_check_launch("rms_scale_kernel");
+}
+
+// ragged batch: xp (B, Lp) = wrap pad to a multiple of 100 + reflect pad 200 + scale by c[b] (wrap_pad_reflect_kernel);
+// needs 200 < lens[b] and Lp >= ceil(lens[b] / 100) * 100 + 400 for every b
+CMGAN_API int cmgan_wrap_pad_reflect_varlen(const float* x, long long ldx, int B, const int* lens, const float* c, float* xp, int Lp, void* stream) {
+    CMGAN_REQUIRE(x && lens && c && xp && Lp > 0, "cmgan_wrap_pad_reflect_varlen: bad arguments");
+    if (B == 0) return 0;
+    dim3 grid(cdiv(Lp, 256), B);
+    wrap_pad_reflect_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x, ldx, lens, c, xp, Lp);
+    return cmgan_check_launch("wrap_pad_reflect_kernel");
 }
 
 // xp (B, Lp): reflect-padded (200 each side) and scaled by c[b] (c may be null); Lp >= L + 400, zero filled beyond
@@ -404,6 +473,16 @@ CMGAN_API int cmgan_ola(const float* frames, int B, int T, const float* inv_env,
     dim3 grid(cdiv((long)HOP * (T - 1), 256), B);
     ola_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(frames, T, inv_env, c_div, y, ldy);
     return cmgan_check_launch("ola_kernel");
+}
+
+// ragged batch: frames (B*T, 400), utterance b has nframes[b] frames (2 <= nframes[b] <= T); win_sq = 400 doubles (squared Hamming window)
+CMGAN_API int cmgan_ola_varlen(const float* frames, int B, int T, const int* nframes, const double* win_sq, const float* c_div, float* y,
+                               long long ldy, void* stream) {
+    CMGAN_REQUIRE(frames && nframes && win_sq && y && T >= 2, "cmgan_ola_varlen: bad arguments");
+    if (B == 0) return 0;
+    dim3 grid(cdiv((long)HOP * (T - 1), 256), B);
+    ola_varlen_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(frames, T, nframes, win_sq, c_div, y, ldy);
+    return cmgan_check_launch("ola_varlen_kernel");
 }
 
 CMGAN_API int cmgan_ola_bwd(const float* dy, long long lddy, int B, int T, const float* inv_env, float* dframes, void* stream) {

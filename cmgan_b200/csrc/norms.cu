@@ -136,13 +136,22 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const float* __restrict__ d
 
 // ---------------------------------------------------------------- group statistics (InstanceNorm2d / BatchNorm1d)
 // sums[(grp*C + c)*2 + {0,1}] += sum x, sum x^2 over the rows of group grp.  Block = one chunk of rows of
-// one group; thread = (row-subgroup, channel).
+// one group; thread = (row-subgroup, channel).  frames (optional, ragged batch): group grp covers its first frames[grp] * rows_per_frame
+// rows only (the rows of padded frames are never read).
+template <bool VAR>
+__device__ __forceinline__ long group_rows(long rows_per_group, const int* __restrict__ frames, long rows_per_frame, int grp) {
+    return VAR ? (long)varlen_frames(frames, grp, (int)(rows_per_group / rows_per_frame)) * rows_per_frame : rows_per_group;
+}
+
+template <bool VAR>
 __global__ void norm_stats_kernel(const float* __restrict__ x, long ldx, long rows_per_group, int C, int chunk,
-                                  double* __restrict__ sums) {
+                                  double* __restrict__ sums, const int* __restrict__ frames, long rows_per_frame) {
     extern __shared__ double sm[];
     int grp = blockIdx.y;
+    const long rows = group_rows<VAR>(rows_per_group, frames, rows_per_frame, grp);
     long r_beg = (long)blockIdx.x * chunk;
-    long r_end = r_beg + chunk < rows_per_group ? r_beg + chunk : rows_per_group;
+    if (VAR && r_beg >= rows) return;
+    long r_end = r_beg + chunk < rows ? r_beg + chunk : rows;
     int c = threadIdx.x % C, rg = threadIdx.x / C, nrg = blockDim.x / C;
     float s = 0.f, q = 0.f;
     const float* base = x + ((long)grp * rows_per_group) * ldx + c;
@@ -159,11 +168,15 @@ __global__ void norm_stats_kernel(const float* __restrict__ x, long ldx, long ro
 }
 
 // same, 128-bit loads: thread = (row-subgroup, 4 channels); C, ldx multiples of 4, x 16-byte aligned
-__global__ void norm_stats4_kernel(const float* __restrict__ x, long ldx, long rows_per_group, int C, int chunk, double* __restrict__ sums) {
+template <bool VAR>
+__global__ void norm_stats4_kernel(const float* __restrict__ x, long ldx, long rows_per_group, int C, int chunk, double* __restrict__ sums,
+                                   const int* __restrict__ frames, long rows_per_frame) {
     __shared__ float sm[256][8];
     const int grp = blockIdx.y, cv = C / 4;
+    const long rows = group_rows<VAR>(rows_per_group, frames, rows_per_frame, grp);
     const long r_beg = (long)blockIdx.x * chunk;
-    const long r_end = r_beg + chunk < rows_per_group ? r_beg + chunk : rows_per_group;
+    if (VAR && r_beg >= rows) return;
+    const long r_end = r_beg + chunk < rows ? r_beg + chunk : rows;
     const int c4 = threadIdx.x % cv, rg = threadIdx.x / cv, nrg = blockDim.x / cv;
     float4 s = make_float4(0.f, 0.f, 0.f, 0.f), q = s;
     const float* base = x + ((long)grp * rows_per_group) * ldx + c4 * 4;
@@ -191,14 +204,16 @@ __global__ void norm_stats4_kernel(const float* __restrict__ x, long ldx, long r
 // mode 1: eval-mode BatchNorm: running statistics
 // outputs per (grp, c): scale = gamma*rstd, shift = beta - mean*scale, mean, rstd (table stride = tstride)
 // when running_mean != null and mode 0: running <- (1-mom)*running + mom*(mean, unbiased var) (BatchNorm1d train)
+// frames (optional, mode 0, ragged batch): group grp averages over n_g = frames[grp] * n rows (n = rows per frame, frames[grp] <= T)
 __global__ void norm_finalize_kernel(const double* __restrict__ sums, long n, int G, int C, int mode,
                                      const float* __restrict__ gamma, const float* __restrict__ beta,
                                      float* __restrict__ running_mean, float* __restrict__ running_var, float momentum,
                                      float* __restrict__ scale, float* __restrict__ shift, float* __restrict__ mean_out,
-                                     float* __restrict__ rstd_out, long tstride) {
+                                     float* __restrict__ rstd_out, long tstride, const int* __restrict__ frames, int T) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= G * C) return;
     int grp = i / C, c = i % C;
+    if (frames) n *= varlen_frames(frames, grp, T);
     float mean, var;
     if (mode == 1) { mean = running_mean[c]; var = running_var[c]; }
     else {
@@ -503,21 +518,37 @@ CMGAN_API int cmgan_ln_bwd_drop(const float* dy, long long lddy, const float* x,
 static int norm_threads(int C) { return C <= 256 ? 256 : C; }
 
 // sums must be zeroed by the caller (G*C*2 doubles).
-CMGAN_API int cmgan_norm_stats(const float* x, long long ldx, int G, long long rows_per_group, int C, double* sums, void* stream) {
+static int norm_stats_launch(const float* x, long long ldx, int G, long long rows_per_group, int C, const int* frames, long long rows_per_frame,
+                             double* sums, void* stream) {
     CMGAN_REQUIRE(x && sums && C >= 1 && C <= 256 && 256 % C == 0, "cmgan_norm_stats: C=%d unsupported", C);
     if (G == 0 || rows_per_group == 0) return 0;
     if (C % 4 == 0 && ldx % 4 == 0 && (((uintptr_t)x) & 15) == 0) {
         const int nrg4 = 256 / (C / 4);
         const int chunk4 = nrg4 * 16;                 // 16 x 128-bit loads per thread; ~1000 blocks on the hot shapes
         dim3 grid4(cdiv(rows_per_group, chunk4), G);
-        norm_stats4_kernel<<<grid4, 256, 0, (cudaStream_t)stream>>>(x, ldx, rows_per_group, C, chunk4, sums);
+        if (frames) norm_stats4_kernel<true><<<grid4, 256, 0, (cudaStream_t)stream>>>(x, ldx, rows_per_group, C, chunk4, sums, frames, rows_per_frame);
+        else norm_stats4_kernel<false><<<grid4, 256, 0, (cudaStream_t)stream>>>(x, ldx, rows_per_group, C, chunk4, sums, nullptr, 1);
         return cmgan_check_launch("norm_stats4_kernel");
     }
     int nrg = 256 / C;
     int chunk = nrg * 64;
     dim3 grid(cdiv(rows_per_group, chunk), G);
-    norm_stats_kernel<<<grid, norm_threads(C), 256 * 2 * sizeof(double), (cudaStream_t)stream>>>(x, ldx, rows_per_group, C, chunk, sums);
+    const size_t smem = 256 * 2 * sizeof(double);
+    if (frames) norm_stats_kernel<true><<<grid, norm_threads(C), smem, (cudaStream_t)stream>>>(x, ldx, rows_per_group, C, chunk, sums, frames, rows_per_frame);
+    else norm_stats_kernel<false><<<grid, norm_threads(C), smem, (cudaStream_t)stream>>>(x, ldx, rows_per_group, C, chunk, sums, nullptr, 1);
     return cmgan_check_launch("norm_stats_kernel");
+}
+
+CMGAN_API int cmgan_norm_stats(const float* x, long long ldx, int G, long long rows_per_group, int C, double* sums, void* stream) {
+    return norm_stats_launch(x, ldx, G, rows_per_group, C, nullptr, 1, sums, stream);
+}
+
+// ragged batch: group g (stride rows_per_group = T * rows_per_frame) covers its first frames[g] * rows_per_frame rows
+CMGAN_API int cmgan_norm_stats_varlen(const float* x, long long ldx, int G, long long rows_per_group, int C, const int* frames,
+                                      long long rows_per_frame, double* sums, void* stream) {
+    CMGAN_REQUIRE(frames && rows_per_frame > 0 && rows_per_group % rows_per_frame == 0,
+                  "cmgan_norm_stats_varlen: rows_per_group must be a multiple of rows_per_frame > 0");
+    return norm_stats_launch(x, ldx, G, rows_per_group, C, frames, rows_per_frame, sums, stream);
 }
 
 CMGAN_API int cmgan_norm_finalize(const double* sums, long long n, int G, int C, int mode, const float* gamma, const float* beta,
@@ -527,7 +558,17 @@ CMGAN_API int cmgan_norm_finalize(const double* sums, long long n, int G, int C,
     CMGAN_REQUIRE(mode == 1 ? (running_mean && running_var) : (sums != nullptr), "cmgan_norm_finalize: missing statistics");
     norm_finalize_kernel<<<cdiv((long)G * C, 128), 128, 0, (cudaStream_t)stream>>>(sums, n, G, C, mode, gamma, beta, running_mean,
                                                                                  running_var, momentum, scale, shift, mean_out,
-                                                                                 rstd_out, tstride);
+                                                                                 rstd_out, tstride, nullptr, 0);
+    return cmgan_check_launch("norm_finalize_kernel");
+}
+
+// InstanceNorm tables of a ragged batch (sums from cmgan_norm_stats_varlen): group g averages over frames[g] * rows_per_frame rows
+CMGAN_API int cmgan_norm_finalize_varlen(const double* sums, const int* frames, long long rows_per_frame, int T, int G, int C, const float* gamma,
+                                         const float* beta, float* scale, float* shift, float* mean_out, float* rstd_out, long long tstride,
+                                         void* stream) {
+    CMGAN_REQUIRE(sums && frames && gamma && beta && scale && shift && rows_per_frame > 0, "cmgan_norm_finalize_varlen: bad arguments");
+    norm_finalize_kernel<<<cdiv((long)G * C, 128), 128, 0, (cudaStream_t)stream>>>(sums, rows_per_frame, G, C, 0, gamma, beta, nullptr, nullptr,
+                                                                                 0.f, scale, shift, mean_out, rstd_out, tstride, frames, T);
     return cmgan_check_launch("norm_finalize_kernel");
 }
 

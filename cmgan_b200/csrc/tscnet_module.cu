@@ -105,6 +105,8 @@ struct Run {
     bool dry;
     int precision;
     cudaStream_t st;
+    const int* frames = nullptr;    // ragged batch: valid frames per batch item (device), null = every item has all T frames
+    int T = 0;
     int rc = 0;
 
     const float* w(const std::string& key) const {
@@ -172,6 +174,11 @@ void inst_norm_site(Run& r, const float* x, long long ldx, int G, long long rows
     double* s = sums;
     sums += (size_t)G * Cn * 2;
     if (!r.live()) return;
+    if (r.frames) {         // a group's statistics span its valid frames only; rows / T rows per frame (F, F2 or 2 F2 at the sites below)
+        r.ok(cmgan_norm_stats_varlen(x, ldx, G, rows, Cn, r.frames, rows / r.T, s, r.st));
+        r.ok(cmgan_norm_finalize_varlen(s, r.frames, rows / r.T, r.T, G, Cn, gamma, beta, t.scale, t.shift, t.mean, t.rstd, t.width, r.st));
+        return;
+    }
     r.ok(cmgan_norm_stats(x, ldx, G, rows, Cn, s, r.st));
     r.ok(cmgan_norm_finalize(s, rows, G, Cn, 0, gamma, beta, nullptr, nullptr, 0.f, t.scale, t.shift, t.mean, t.rstd, t.width, r.st));
 }
@@ -243,7 +250,11 @@ void conformer(Run& r, const float* x, float* y, const std::string& p, int B, in
     float* lse = r.alloc((size_t)M * 4);
     if (r.live()) {
         const float* E = r.w(p + "attn.fn.rel_pos_emb.weight");
-        r.ok(r.precision == 1 ? cmgan_attention_fwd_tf32(qkv, E, B, T, F2, axis, ctx, lse, r.st) : cmgan_attention_fwd(qkv, E, B, T, F2, axis, ctx, lse, r.st));
+        if (r.frames)
+            r.ok(r.precision == 1 ? cmgan_attention_fwd_tf32_varlen(qkv, E, B, T, F2, axis, r.frames, ctx, lse, r.st)
+                                  : cmgan_attention_fwd_varlen(qkv, E, B, T, F2, axis, r.frames, ctx, lse, r.st));
+        else
+            r.ok(r.precision == 1 ? cmgan_attention_fwd_tf32(qkv, E, B, T, F2, axis, ctx, lse, r.st) : cmgan_attention_fwd(qkv, E, B, T, F2, axis, ctx, lse, r.st));
     }
     float* x2 = r.alloc((size_t)M * C);
     Gemm(ctx, C, r.w(p + "attn.fn.to_out.weight"), 0, 1, C, r.w(p + "attn.fn.to_out.bias"), x2, C, M, C, C).residual(x1, C).run(r);
@@ -257,7 +268,10 @@ void conformer(Run& r, const float* x, float* y, const std::string& p, int B, in
     Tabs bn = make_tabs(r, 1, 2 * C);
     float* dsw = r.alloc((size_t)M * 2 * C);
     if (r.live()) {
-        r.ok(cmgan_glu_dwconv_fwd(g, r.w(p + "conv.net.4.conv.weight"), r.w(p + "conv.net.4.conv.bias"), B, T, F2, axis, d, nullptr, r.st));
+        if (r.frames)
+            r.ok(cmgan_glu_dwconv_fwd_varlen(g, r.w(p + "conv.net.4.conv.weight"), r.w(p + "conv.net.4.conv.bias"), B, T, F2, axis, r.frames, d, r.st));
+        else
+            r.ok(cmgan_glu_dwconv_fwd(g, r.w(p + "conv.net.4.conv.weight"), r.w(p + "conv.net.4.conv.bias"), B, T, F2, axis, d, nullptr, r.st));
         // eval: BatchNorm1d folds to scale / shift from the running statistics (mode 1; they are only read)
         r.ok(cmgan_norm_finalize(nullptr, M, 1, 2 * C, 1, r.w(p + "conv.net.5.weight"), r.w(p + "conv.net.5.bias"),
                                  const_cast<float*>(r.w(p + "conv.net.5.running_mean")), const_cast<float*>(r.w(p + "conv.net.5.running_var")), 0.1f,
@@ -362,8 +376,13 @@ CMGAN_API long long cmgan_tscnet_workspace_bytes(int B, int T, int F, int precis
     return (long long)r.peak + 256;
 }
 
-CMGAN_API int cmgan_tscnet_fwd(const float* params, const float* x, long long sxb, long long sxc, long long sxt, long long sxf, int B, int T, int F,
-                               float* final_real, float* final_imag, void* workspace, long long workspace_bytes, int precision, void* stream) {
+// Ragged batch (inference on clips of different lengths in one pass): frames = device int[B], 1 <= frames[b] <= T.  For t < frames[b] the
+// outputs equal cmgan_tscnet_fwd on x[b, :, :frames[b]] alone; rows t >= frames[b] of x are never read by a valid row (the convolutions
+// are causal in time; attention, the depthwise convolution and the InstanceNorm statistics stop at frames[b]) and their outputs are
+// unspecified.  frames == NULL is cmgan_tscnet_fwd.  The workspace is the one cmgan_tscnet_workspace_bytes(B, T, F, precision) gives.
+CMGAN_API int cmgan_tscnet_fwd_varlen(const float* params, const float* x, long long sxb, long long sxc, long long sxt, long long sxf, int B, int T,
+                                      int F, const int* frames, float* final_real, float* final_imag, void* workspace, long long workspace_bytes,
+                                      int precision, void* stream) {
     CMGAN_REQUIRE(params && x && final_real && final_imag && workspace, "cmgan_tscnet_fwd: null pointer");
     CMGAN_REQUIRE(B > 0 && T > 0 && F == NFEAT, "cmgan_tscnet_fwd: expected x of shape (B, 2, T, %d), got B=%d T=%d F=%d", NFEAT, B, T, F);
     CMGAN_REQUIRE(precision == 0 || precision == 1, "cmgan_tscnet_fwd: precision must be 0 (fp32) or 1 (tf32)");
@@ -372,6 +391,13 @@ CMGAN_API int cmgan_tscnet_fwd(const float* params, const float* x, long long sx
     Run r;
     r.P = params; r.ws = static_cast<char*>(workspace); r.cap = (size_t)workspace_bytes; r.dry = false; r.precision = precision;
     r.st = (cudaStream_t)stream;
+    r.frames = frames; r.T = T;
     forward(r, x, sxb, sxc, sxt, sxf, B, T, F, final_real, final_imag);
     return r.rc;
+}
+
+CMGAN_API int cmgan_tscnet_fwd(const float* params, const float* x, long long sxb, long long sxc, long long sxt, long long sxf, int B, int T, int F,
+                               float* final_real, float* final_imag, void* workspace, long long workspace_bytes, int precision, void* stream) {
+    return cmgan_tscnet_fwd_varlen(params, x, sxb, sxc, sxt, sxf, B, T, F, nullptr, final_real, final_imag, workspace, workspace_bytes, precision,
+                                   stream);
 }

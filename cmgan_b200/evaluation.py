@@ -6,9 +6,10 @@ the signal's own head, fold files longer than ``cut_len`` into a batch, STFT -> 
 is absent here; 16-bit PCM, 32-bit float and 32-bit PCM files are read to float32 in [-1, 1) exactly as torchaudio does, float32 is
 written like soundfile's default for float input would be on a FLOAT-subtype file -- pass ``subtype='PCM_16'`` for 16-bit output).
 
-``enhance_files`` is the throughput front-end for the config-5 sweep: files are bucketed by padded length (InstanceNorm statistics span
-the whole (T, F) plane, so only clips of identical length can share a batch without changing any output) and every bucket goes through
-the network as one batch.
+``enhance_files`` is the throughput front-end: files of different lengths share one forward pass as a ragged batch (signal.plan_ragged sorts
+them by length and cuts groups of at most ``max_batch``; signal.enhance_ragged pads each group to its longest clip and TSCNet reads only
+each clip's own frames -- the convolutions are causal in time, attention, the depthwise convolution and the InstanceNorm statistics stop at
+each clip's length), so every file gets its per-file result.  ``evaluation`` enhances through it and scores file by file.
 """
 from __future__ import annotations
 
@@ -77,37 +78,34 @@ def enhance_one_track(model, audio_path: str, saved_dir: Optional[str], cut_len:
 
 @torch.no_grad()
 def enhance_files(model, paths: Sequence[str], cut_len: int = SR * 16, max_batch: int = 16) -> Dict[str, np.ndarray]:
-    """Enhance many files with identical-length clips batched together (bit-for-bit the per-file results: nothing is padded or mixed).
-    Files longer than ``cut_len`` take the reference's folding path one at a time."""
+    """Enhance many files -> {path: enhanced (length,) float32}, the per-file results of ``enhance_one_track``.  Files up to ``cut_len``
+    go through ragged batches of at most ``max_batch`` clips of mixed lengths (signal.plan_ragged / signal.enhance_ragged); longer files
+    take the reference's folding path one at a time."""
     dev = next(model.parameters()).device
-    waves, buckets = {}, {}
+    paths = list(paths)
+    waves = []
     for p in paths:
         x, sr = read_wav(p)
         assert sr == SR
-        waves[p] = x[:1]
-        L = x.size(-1)
-        key = L if int(np.ceil(L / 100)) * 100 <= cut_len else ("solo", p)
-        buckets.setdefault(key, []).append(p)
+        waves.append(x[0])
+    batches, solo = signal.plan_ragged([w.numel() for w in waves], max_batch=max_batch, cut_len=cut_len)
     out: Dict[str, np.ndarray] = {}
-    for key, group in buckets.items():
-        if isinstance(key, tuple):
-            out[group[0]] = signal.enhance(model, waves[group[0]].to(dev), cut_len=cut_len).cpu().numpy()
-            continue
-        for i in range(0, len(group), max_batch):
-            part = group[i:i + max_batch]
-            batch = torch.cat([waves[p] for p in part], dim=0).to(dev)
-            est = signal.enhance_batch(model, batch)
-            for p, e in zip(part, est):
-                out[p] = e.cpu().numpy()
+    for i in solo:
+        out[paths[i]] = signal.enhance(model, waves[i][None].to(dev), cut_len=cut_len).cpu().numpy()
+    for idx in batches:
+        est = signal.enhance_ragged(model, [waves[i] for i in idx], cut_len=cut_len)
+        for i, e in zip(idx, est):
+            out[paths[i]] = e.cpu().numpy()
     return out
 
 
 @torch.no_grad()
 def evaluation(model, noisy_dir: str, clean_dir: str, save_tracks: bool, saved_dir: str,
-               metrics: Optional[Callable[[np.ndarray, np.ndarray], Sequence[float]]] = None, cut_len: int = SR * 16):
-    """reference evaluation.py:60-97 with an already-loaded ``model``: enhance every file of ``noisy_dir`` in natural order, score it against
-    the file of the same name in ``clean_dir`` with ``metrics(clean, enhanced) -> sequence`` (default: the PESQ-free pair SSNR, STOI from
-    cmgan_b200.metrics on the GPU) and return the per-metric averages."""
+               metrics: Optional[Callable[[np.ndarray, np.ndarray], Sequence[float]]] = None, cut_len: int = SR * 16, max_batch: int = 16):
+    """reference evaluation.py:60-97 with an already-loaded ``model``: enhance every file of ``noisy_dir`` (``enhance_files``: ragged batches
+    of up to ``max_batch`` files, the per-file results), then in natural order save it and score it against the file of the same name in
+    ``clean_dir`` with ``metrics(clean, enhanced) -> sequence`` (default: the PESQ-free pair SSNR, STOI from cmgan_b200.metrics on the GPU);
+    returns the per-metric averages."""
     model.eval()
     if save_tracks and not os.path.exists(saved_dir):
         os.mkdir(saved_dir)
@@ -118,9 +116,13 @@ def evaluation(model, noisy_dir: str, clean_dir: str, save_tracks: bool, saved_d
         def metrics(clean, est):
             return gpu_metrics.ssnr_stoi(torch.from_numpy(clean).to(dev), torch.from_numpy(est).to(dev))
     names = natural_sorted(os.listdir(noisy_dir))
+    enhanced = enhance_files(model, [os.path.join(noisy_dir, name) for name in names], cut_len=cut_len, max_batch=max_batch)
     total = None
     for name in names:
-        est_audio, length = enhance_one_track(model, os.path.join(noisy_dir, name), saved_dir, cut_len, 400, 100, save_tracks)
+        est_audio = enhanced[os.path.join(noisy_dir, name)]
+        length = len(est_audio)
+        if save_tracks:
+            write_wav(os.path.join(saved_dir, name), est_audio, SR)
         clean, sr = read_wav(os.path.join(clean_dir, name))
         assert sr == SR
         m = np.asarray(metrics(clean[0].numpy()[:length], est_audio), dtype=np.float64)

@@ -217,11 +217,16 @@ class TSCNet(nn.Module):
         G = {k: torch.zeros_like(named[k]) for k in self._param_keys}
         return G, tuple(G[k] if named[k].requires_grad else None for k in self._param_keys)
 
-    def forward(self, x: torch.Tensor):
+    def forward(self, x: torch.Tensor, frames=None):
+        """``frames`` (optional): ragged batch for inference -- item b of the padded input holds frames[b] valid frames (host-side
+        sequence or tensor of B ints, 1 <= frames[b] <= T).  Output frames t < frames[b] equal ``forward(x[b:b+1, :, :frames[b]])``; the
+        rest are unspecified (the padded input frames may hold anything and are never read by a valid frame)."""
         if not x.is_cuda:
             raise RuntimeError("cmgan_b200.TSCNet runs on CUDA only (no CPU fallback)")
         if x.dtype != torch.float32:
             raise RuntimeError("cmgan_b200.TSCNet expects float32 input")
+        if frames is not None:
+            frames = self._ragged_frames(x, frames)
         if self.training:
             self._step += 1
             torch._foreach_add_([b for k, b in self.named_buffers() if k.endswith("num_batches_tracked")], 1)   # bookkeeping only
@@ -235,7 +240,26 @@ class TSCNet(nn.Module):
                 self._pack_sig = sig
             ops.PACK_CACHE = self._pack
             try:
-                return _TSCNetFn.apply(x, self, self.training, self.seed * 7919 + self._step, *params)
+                return self._run(x, params, frames)
             finally:
                 ops.PACK_CACHE = None
-        return _TSCNetFn.apply(x, self, self.training, self.seed * 7919 + self._step, *params)
+        return self._run(x, params, frames)
+
+    def _run(self, x, params, frames):
+        if frames is None:
+            return _TSCNetFn.apply(x, self, self.training, self.seed * 7919 + self._step, *params)
+        return tscnet_fwd(x, self._tensor_dict(), False, 0, None, frames)
+
+    def _ragged_frames(self, x: torch.Tensor, frames) -> torch.Tensor:
+        """validate host-side frame counts of a ragged batch, then upload them (device int32 (B,))"""
+        if self.training or torch.is_grad_enabled():
+            raise ValueError("TSCNet.forward(x, frames): ragged batches are inference only (model.eval() under torch.no_grad())")
+        if ops.PRECISION == 1 and ops.ATTN_TC:
+            raise ValueError("TSCNet.forward(x, frames): the tcgen05 attention forward (CMGAN_ATTN_TC=1) has no ragged-batch variant")
+        B, T = x.shape[0], x.shape[2]
+        n = torch.as_tensor(frames).detach().to("cpu", torch.int64).reshape(-1)
+        if n.numel() != B:
+            raise ValueError(f"TSCNet.forward(x, frames): expected {B} frame counts, got {n.numel()}")
+        if B and (int(n.min()) < 1 or int(n.max()) > T):
+            raise ValueError(f"TSCNet.forward(x, frames): frame counts must lie in [1, {T}], got [{int(n.min())}, {int(n.max())}]")
+        return n.to(torch.int32).to(x.device)

@@ -40,8 +40,9 @@ def workspace_bytes(B: int, T: int, F: int, precision: int) -> int:
     return n
 
 
-def tscnet_forward(flat: torch.Tensor, x: torch.Tensor, precision: int = 1, workspace: torch.Tensor = None):
-    """x (B, 2, T, F) on the GPU, any strides -> (final_real, final_imag), each (B, 1, T, F)"""
+def tscnet_forward(flat: torch.Tensor, x: torch.Tensor, precision: int = 1, workspace: torch.Tensor = None, frames: torch.Tensor = None):
+    """x (B, 2, T, F) on the GPU, any strides -> (final_real, final_imag), each (B, 1, T, F).
+    ``frames`` (optional, device int32 (B,)): ragged batch through ``cmgan_tscnet_fwd_varlen`` (frames t >= frames[b] unspecified)"""
     assert x.is_cuda and flat.is_cuda and x.dtype == torch.float32 and x.dim() == 4 and x.shape[1] == 2
     B, _, T, F = x.shape
     if workspace is None:
@@ -49,6 +50,11 @@ def tscnet_forward(flat: torch.Tensor, x: torch.Tensor, precision: int = 1, work
     fr = torch.empty(B, 1, T, F, device=x.device)
     fi = torch.empty(B, 1, T, F, device=x.device)
     sb, sc, st, sf = x.stride()
+    if frames is not None:
+        assert frames.is_cuda and frames.dtype == torch.int32 and frames.numel() == B and frames.is_contiguous()
+        lib().call("cmgan_tscnet_fwd_varlen", flat.data_ptr(), x.data_ptr(), sb, sc, st, sf, B, T, F, frames.data_ptr(), fr.data_ptr(),
+                   fi.data_ptr(), workspace.data_ptr(), workspace.numel(), precision, torch.cuda.current_stream().cuda_stream)
+        return fr, fi
     lib().call("cmgan_tscnet_fwd", flat.data_ptr(), x.data_ptr(), sb, sc, st, sf, B, T, F, fr.data_ptr(), fi.data_ptr(), workspace.data_ptr(),
                workspace.numel(), precision, torch.cuda.current_stream().cuda_stream)
     return fr, fi

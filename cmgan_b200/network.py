@@ -28,17 +28,18 @@ def _act_code():
     return 1 | (16 if ops.PRECISION == 1 else 0)       # PReLU (+ round to tf32 for the tensor-core consumers)
 
 
-def _norm_prelu_to(raw, ldr, G, rows, gamma, beta, slope, dst, ldd, sums: _Sums, dev) -> _Tabs:
+def _norm_prelu_to(raw, ldr, G, rows, gamma, beta, slope, dst, ldd, sums: _Sums, dev, frames=None, T=None) -> _Tabs:
     """InstanceNorm2d(affine) + PReLU of a raw (M, 64) tensor, materialised into ``dst`` (ref: generator.py:35-37)"""
     tab = _Tabs(G, C, dev)
-    _inst_norm_site(raw, ldr, G, rows, C, gamma, beta, tab, 0, None, sums)
+    _inst_norm_site(raw, ldr, G, rows, C, gamma, beta, tab, 0, None, sums, frames, T)
     call("cmgan_norm_apply", raw, ldr, G, rows, C, _act_code(), tab.scale, tab.shift, C, slope, dst, ldd)
     return tab
 
 
-def dense_block_fwd(cat, P, p, B, T, Fw, sums: _Sums):
+def dense_block_fwd(cat, P, p, B, T, Fw, sums: _Sums, frames=None):
     """DilatedDenseNet (ref: generator.py:39-47).  ``cat`` slot 4 holds the (activated) block input; returns the per-layer raw
-    conv outputs and normalisation tables.  Layer i leaves act(out_i) in slot 4 - i."""
+    conv outputs and normalisation tables.  Layer i leaves act(out_i) in slot 4 - i.  The convolutions are causal in time, so with
+    ``frames`` (ragged batch) only the InstanceNorm statistics need to know the lengths."""
     dev = cat.device
     M, rows = B * T * Fw, T * Fw
     raws, tabs = [], []
@@ -48,7 +49,7 @@ def dense_block_fwd(cat, P, p, B, T, Fw, sums: _Sums):
         gemm(A=(cat, c0), lda=CAT, W=P[f"{p}.conv{i}.weight"], sb_tap=1, sb_k=6, sb_n=Cin * 6, bias=P[f"{p}.conv{i}.bias"], C=raw, ldc=C,
              M=M, N=C, Cin=Cin, taps=_dense_taps(dil), conv=dict(OH=T, OW=Fw, IH=T, IW=Fw))
         tabs.append(_norm_prelu_to(raw, C, B, rows, P[f"{p}.norm{i}.weight"], P[f"{p}.norm{i}.bias"], P[f"{p}.prelu{i}.weight"], (cat, co), CAT,
-                                   sums, dev))
+                                   sums, dev, frames, T))
         raws.append(raw)
     return raws, tabs
 
@@ -73,8 +74,12 @@ def _sums_size(B):
     return (16 * C + 2) * B * 2 + 8 * 2 * C * 2 + 64
 
 
-def tscnet_fwd(x, P, training: bool, seed: int, save: Optional[dict]):
-    """TSCNet.forward (ref: generator.py:174-196).  x (B, 2, T, F) any strides -> final_real, final_imag (B, 1, T, F)."""
+def tscnet_fwd(x, P, training: bool, seed: int, save: Optional[dict], frames=None):
+    """TSCNet.forward (ref: generator.py:174-196).  x (B, 2, T, F) any strides -> final_real, final_imag (B, 1, T, F).
+    ``frames`` (inference only): ragged batch, device int32 (B,) with 1 <= frames[b] <= T.  For t < frames[b] the outputs equal this
+    function on x[b:b+1, :, :frames[b]] alone; the rows of padded frames are never read by a valid row and their outputs are unspecified."""
+    if frames is not None and (training or save is not None):
+        raise ValueError("tscnet_fwd: ragged batches (frames) are inference only")
     dev = x.device
     B, two, T, F = x.shape
     assert two == 2 and F % 2 == 1, "expected x of shape (B, 2, T, F) with odd F"
@@ -88,28 +93,28 @@ def tscnet_fwd(x, P, training: bool, seed: int, save: Optional[dict]):
     raw0 = _empty(M, C, dev=dev)
     call("cmgan_head_conv", x, xs[0], xs[1], xs[2], xs[3], B, T, F, P[pe + ".conv_1.0.weight"], P[pe + ".conv_1.0.bias"], raw0, C)
     tab0 = _norm_prelu_to(raw0, C, B, T * F, P[pe + ".conv_1.1.weight"], P[pe + ".conv_1.1.bias"], P[pe + ".conv_1.2.weight"], (catE, 4 * C), CAT,
-                          sums, dev)
-    rawsE, tabsE = dense_block_fwd(catE, P, pe + ".dilated_dense", B, T, F, sums)
+                          sums, dev, frames, T)
+    rawsE, tabsE = dense_block_fwd(catE, P, pe + ".dilated_dense", B, T, F, sums, frames)
     e2 = _empty(M2, C, dev=dev)
     gemm(A=catE, lda=CAT, W=P[pe + ".conv_2.0.weight"], sb_tap=1, sb_k=3, sb_n=3 * C, bias=P[pe + ".conv_2.0.bias"], C=e2, ldc=C, M=M2, N=C, Cin=C,
          taps=_W3, conv=dict(OH=T, OW=F2, IH=T, IW=F, mul_x=2))
     h = _empty(M2, C, dev=dev)
     tab2 = _Tabs(B, C, dev)
-    _inst_norm_site(e2, C, B, T * F2, C, P[pe + ".conv_2.1.weight"], P[pe + ".conv_2.1.bias"], tab2, 0, None, sums)
+    _inst_norm_site(e2, C, B, T * F2, C, P[pe + ".conv_2.1.weight"], P[pe + ".conv_2.1.bias"], tab2, 0, None, sums, frames, T)
     call("cmgan_norm_apply", e2, C, B, T * F2, C, 1, tab2.scale, tab2.shift, C, P[pe + ".conv_2.2.weight"], h, C)
     # ---- 4 x TSCB (ref: generator.py:92-99)
     conf_saves = []
     for i in range(1, 5):
         for axis, name in ((0, "time_conformer"), (1, "freq_conformer")):
             sv = {} if save is not None else None
-            h = conformer_fwd(h, P, f"TSCB_{i}.{name}", B, T, F2, axis, training, seed, (i - 1) * 2 + axis, sums, sv)
+            h = conformer_fwd(h, P, f"TSCB_{i}.{name}", B, T, F2, axis, training, seed, (i - 1) * 2 + axis, sums, sv, frames)
             conf_saves.append(sv)
     # ---- decoders (ref: generator.py:122-156)
     dec = {}
     for pd in ("mask_decoder", "complex_decoder"):
         cat = _empty(M2, CAT, dev=dev)
         call("cmgan_copy_rows_operand", h, C, (cat, 4 * C), CAT, M2, C)         # operand of the decoder's first convolution
-        raws, tabs = dense_block_fwd(cat, P, pd + ".dense_block", B, T, F2, sums)
+        raws, tabs = dense_block_fwd(cat, P, pd + ".dense_block", B, T, F2, sums, frames)
         sp = _empty(M2, 2 * C, dev=dev)      # == (B, T, 2*F2, 64): the sub-pixel shuffle is a free reinterpretation
         gemm(A=cat, lda=CAT, W=P[pd + ".sub_pixel.conv.weight"], sb_tap=1, sb_k=3, sb_n=3 * C, bias=P[pd + ".sub_pixel.conv.bias"], C=sp, ldc=2 * C,
              M=M2, N=2 * C, Cin=C, taps=_W3, conv=dict(OH=T, OW=F2, IH=T, IW=F2))
@@ -118,9 +123,9 @@ def tscnet_fwd(x, P, training: bool, seed: int, save: Optional[dict]):
     m1 = _empty(M, dev=dev)
     call("cmgan_rowdot_fwd", dec[pm]["sp"], B, T, F, 1, None, None, None, P[pm + ".conv_1.weight"], P[pm + ".conv_1.bias"], m1)
     tabM = _Tabs(B, 1, dev)
-    _inst_norm_site(m1, 1, B, T * F, 1, P[pm + ".norm.weight"], P[pm + ".norm.bias"], tabM, 0, None, sums)
+    _inst_norm_site(m1, 1, B, T * F, 1, P[pm + ".norm.weight"], P[pm + ".norm.bias"], tabM, 0, None, sums, frames, T)
     tabC = _Tabs(B, C, dev)
-    _inst_norm_site(dec[pc]["sp"], C, B, T * 2 * F2, C, P[pc + ".norm.weight"], P[pc + ".norm.bias"], tabC, 0, None, sums)
+    _inst_norm_site(dec[pc]["sp"], C, B, T * 2 * F2, C, P[pc + ".norm.weight"], P[pc + ".norm.bias"], tabC, 0, None, sums, frames, T)
     cplx = _empty(M, 2, dev=dev)
     call("cmgan_rowdot_fwd", dec[pc]["sp"], B, T, F, 2, tabC.scale, tabC.shift, P[pc + ".prelu.weight"], P[pc + ".conv.weight"],
          P[pc + ".conv.bias"], cplx)

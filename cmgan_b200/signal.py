@@ -8,7 +8,7 @@ inverse basis followed by overlap-add.  Both run in exact fp32 FFMA (0.1 GFLOP p
 from __future__ import annotations
 
 import math
-from typing import Dict, Tuple
+from typing import Dict, List, Sequence, Tuple
 
 import torch
 
@@ -50,6 +50,14 @@ def _inv_basis(dev) -> torch.Tensor:
     return _CACHE[key]
 
 
+def _window_sq(dev) -> torch.Tensor:
+    """(400,) float64 squared analysis window: the terms _inv_envelope sums (the ragged overlap-add sums them on the GPU)"""
+    key = ("wsq", dev)
+    if key not in _CACHE:
+        _CACHE[key] = (_window64() ** 2).contiguous().to(dev)
+    return _CACHE[key]
+
+
 def _inv_envelope(T: int, dev) -> torch.Tensor:
     """1 / sum_t w^2[n + 200 - 100 t] for n < 100 (T - 1)"""
     key = ("env", T, dev)
@@ -83,6 +91,13 @@ def stft_compress(wav: torch.Tensor, scale: torch.Tensor = None) -> torch.Tensor
     Lp = ((L + N_FFT + HOP - 1) // HOP) * HOP
     xp = torch.empty(B, Lp, device=dev)
     call("cmgan_pad_reflect", wav, wav.stride(0), B, L, scale, xp, Lp)
+    return _stft_padded(xp, T)
+
+
+def _stft_padded(xp: torch.Tensor, T: int) -> torch.Tensor:
+    """(B, Lp) padded waveform (Lp a multiple of 100, >= 100 (T - 1) + 400) -> power-compressed (B, 2, T, F) as the (B, 2, F, T) view"""
+    dev = xp.device
+    B, Lp = xp.shape
     S = torch.empty(B * T, 2 * NF, device=dev)
     gemm(A=xp, lda=HOP, W=_fwd_basis(dev), sb_k=2 * NF, sb_n=1, C=S, ldc=2 * NF, M=B * T, N=2 * NF, Cin=N_FFT, taps=[(0, 0)],
          conv=dict(OH=1, OW=T, IH=1, IW=Lp // HOP), precision=0)      # the DFTs stay exact fp32
@@ -182,3 +197,86 @@ def enhance(model, noisy: torch.Tensor, cut_len: int = 16000 * 16) -> torch.Tens
     fr, fi = model(spec)
     audio = uncompress_istft(fr, fi, cb)
     return audio.reshape(-1)[:length]
+
+
+# ---------------------------------------------------------------------------------------------------------- ragged batches
+MAX_CAT_ELEMS = 2 ** 31     # the encoder's (B T F, 320) concat buffer is indexed with 32-bit element counts
+
+
+def clip_frames(length: int) -> int:
+    """STFT frames of a clip of ``length`` samples after the wrap padding to a multiple of 100 (evaluation.py:25-29)"""
+    return int(math.ceil(length / HOP)) + 1
+
+
+def plan_ragged(lengths: Sequence[int], max_batch: int = 16, cut_len: int = 16000 * 16) -> Tuple[List[List[int]], List[int]]:
+    """Batch plan for ``enhance_ragged``: -> (batches, solo), lists of indices into ``lengths``.
+    Clips whose wrap-padded length exceeds ``cut_len`` go to ``solo`` (the folding path of ``enhance``, one at a time).  The others are
+    sorted by length and cut into consecutive groups of at most ``max_batch`` clips, so a batch pads little; a group also stops before
+    B * T_max * 201 * 320 reaches 2^31 (the encoder's concat buffer).  Clips of 200 samples or fewer are rejected: the reflect padding
+    of the STFT needs more."""
+    if max_batch < 1:
+        raise ValueError("plan_ragged: max_batch must be >= 1")
+    for i, n in enumerate(lengths):
+        if n <= N_FFT // 2:
+            raise ValueError(f"plan_ragged: clip {i} has {n} samples; at least {N_FFT // 2 + 1} are needed")
+    solo = [i for i, n in enumerate(lengths) if int(math.ceil(n / HOP)) * HOP > cut_len]
+    rest = sorted((i for i, n in enumerate(lengths) if int(math.ceil(n / HOP)) * HOP <= cut_len), key=lambda i: (lengths[i], i))
+    batches: List[List[int]] = []
+    cur: List[int] = []
+    for i in rest:
+        t_max = clip_frames(lengths[i])          # sorted ascending: the clip being added is the longest of its group
+        if cur and (len(cur) == max_batch or (len(cur) + 1) * t_max * NF * 320 >= MAX_CAT_ELEMS):
+            batches.append(cur)
+            cur = []
+        cur.append(i)
+    if cur:
+        batches.append(cur)
+    return batches, solo
+
+
+def uncompress_istft_varlen(fr: torch.Tensor, fi: torch.Tensor, nframes: torch.Tensor, c_div: torch.Tensor) -> torch.Tensor:
+    """``uncompress_istft_fwd`` of a ragged batch: utterance b has nframes[b] (device int32) of the T frames; its samples
+    0 .. 100 (nframes[b] - 1) equal those of a run on its frames alone (per-utterance synthesis envelope), the rest are zero"""
+    dev = fr.device
+    B, _, T, F = fr.shape
+    assert F == NF and fi.stride() == fr.stride()
+    s = fr.stride()
+    U = torch.empty(B * T, 2 * NF, device=dev)
+    call("cmgan_uncompress", fr, fi, s[0], s[2], s[3], B, T, U)
+    frames = torch.empty(B * T, N_FFT, device=dev)
+    gemm(A=U, lda=2 * NF, W=_inv_basis(dev), sb_k=N_FFT, sb_n=1, C=frames, ldc=N_FFT, M=B * T, N=N_FFT, Cin=2 * NF, precision=0)
+    y = torch.empty(B, HOP * (T - 1), device=dev)
+    call("cmgan_ola_varlen", frames, B, T, nframes, _window_sq(dev), c_div, y, y.stride(0))
+    return y
+
+
+@torch.no_grad()
+def enhance_ragged(model, waves: Sequence[torch.Tensor], cut_len: int = 16000 * 16) -> List[torch.Tensor]:
+    """Enhance clips of different lengths in one forward pass: each 1-D clip (200 < length, wrap-padded length <= ``cut_len``) gets
+    exactly what ``enhance`` does to one file -- RMS normalisation, wrap padding with its own head, STFT, TSCNet, iSTFT,
+    de-normalisation, truncation -- and the list of enhanced clips (on the model's device) comes back in the input order.
+    The clips are zero-padded to the longest; TSCNet runs on the ragged batch (``TSCNet.forward(x, frames)``)."""
+    if len(waves) == 0:
+        return []
+    lengths = [int(w.numel()) for w in waves]
+    for i, n in enumerate(lengths):
+        if n <= N_FFT // 2 or int(math.ceil(n / HOP)) * HOP > cut_len:
+            raise ValueError(f"enhance_ragged: clip {i} has {n} samples; need {N_FFT // 2} < length and a padded length <= cut_len ({cut_len})")
+    dev = next(model.parameters()).device
+    B = len(waves)
+    x = torch.nn.utils.rnn.pad_sequence([w.reshape(-1) for w in waves], batch_first=True).to(dev, torch.float32).contiguous()
+    nfr = [clip_frames(n) for n in lengths]
+    T = max(nfr)
+    meta = torch.tensor([lengths, nfr], dtype=torch.int32).to(dev)       # one upload: sample counts, frame counts
+    lens, nframes = meta[0], meta[1]
+    c = torch.empty(B, device=dev)
+    call("cmgan_rms_scale_varlen", x, x.stride(0), B, lens, c)
+    Lp = HOP * (T - 1) + N_FFT
+    xp = torch.empty(B, Lp, device=dev)
+    call("cmgan_wrap_pad_reflect_varlen", x, x.stride(0), B, lens, c, xp, Lp)
+    spec = _stft_padded(xp, T).permute(0, 1, 3, 2)
+    fr, fi = model(spec, frames=nfr)
+    if fi.stride() != fr.stride():
+        fr, fi = fr.contiguous(), fi.contiguous()
+    y = uncompress_istft_varlen(fr, fi, nframes, c)
+    return [y[b, :n] for b, n in enumerate(lengths)]

@@ -42,6 +42,8 @@ int cmgan_ln_bwd(const float* dy, long long lddy, const float* x, long long ldx,
 int cmgan_ln_bwd_drop(const float* dy, long long lddy, const float* x, long long ldx, const float* stats, const float* gamma, long long M, const float* res, long long ldr, const float* res2, long long ldr2, float* dx, long long lddx, float* dgamma, float* dbeta, float* dz, long long lddz, float alpha, unsigned long long seed, unsigned int thr, float inv_keep, const unsigned long long* seed_dev, void* stream);
 int cmgan_norm_stats(const float* x, long long ldx, int G, long long rows_per_group, int C, double* sums, void* stream);
 int cmgan_norm_finalize(const double* sums, long long n, int G, int C, int mode, const float* gamma, const float* beta, float* running_mean, float* running_var, float momentum, float* scale, float* shift, float* mean_out, float* rstd_out, long long tstride, void* stream);
+int cmgan_norm_stats_varlen(const float* x, long long ldx, int G, long long rows_per_group, int C, const int* frames, long long rows_per_frame, double* sums, void* stream);
+int cmgan_norm_finalize_varlen(const double* sums, const int* frames, long long rows_per_frame, int T, int G, int C, const float* gamma, const float* beta, float* scale, float* shift, float* mean_out, float* rstd_out, long long tstride, void* stream);
 int cmgan_norm_bwd_reduce(const float* x, long long ldx, const float* dact, long long ldd, int G, long long rows_per_group, int C, int act, const float* scale, const float* shift, const float* mean, const float* rstd, long long tstride, const float* slope, double* S, float* dslope, void* stream);
 int cmgan_norm_bwd_apply(const float* x, long long ldx, const float* dact, long long ldd, int G, long long rows_per_group, int C, int act, int use_batch_stats, const float* scale, const float* shift, const float* mean, const float* rstd, long long tstride, const float* slope, const double* S, float* dx, long long lddx, float* dgamma, float* dbeta, void* stream);
 int cmgan_norm_apply(const float* x, long long ldx, int G, long long rows_per_group, int C, int act, const float* scale, const float* shift, long long tstride, const float* slope, float* y, long long ldy, void* stream);
@@ -50,10 +52,14 @@ int cmgan_copy_rows(const float* src, long long lds, float* dst, long long ldd, 
 int cmgan_copy_rows_operand(const float* src, long long lds, float* dst, long long ldd, long long M, int C, void* stream);
 int cmgan_add_rows(const float* src, long long lds, float* dst, long long ldd, long long M, int C, void* stream);
 
-/* ---- attention with Shaw relative positions (conformer.py:100-131); axis 0 = time sequences, 1 = frequency sequences */
+/* ---- attention with Shaw relative positions (conformer.py:100-131); axis 0 = time sequences, 1 = frequency sequences.
+ * *_varlen (here and below): ragged batch of B items padded to T frames, frames = device int[B], 1 <= frames[b] <= T; rows of padded frames are
+ * never read (they may hold NaN) and their outputs are unspecified. */
 int cmgan_attention_fwd(const float* qkv, const float* E, int B, int T, int F, int axis, float* ctx, float* lse, void* stream);
 int cmgan_attention_fwd_tf32(const float* qkv, const float* E, int B, int T, int F, int axis, float* ctx, float* lse, void* stream);
 int cmgan_attention_fwd_tf32_nbuf(const float* qkv, const float* E, int B, int T, int F, int axis, float* ctx, float* lse, int nbuf, void* stream);
+int cmgan_attention_fwd_varlen(const float* qkv, const float* E, int B, int T, int F, int axis, const int* frames, float* ctx, float* lse, void* stream);
+int cmgan_attention_fwd_tf32_varlen(const float* qkv, const float* E, int B, int T, int F, int axis, const int* frames, float* ctx, float* lse, void* stream);
 int cmgan_attention_fwd_tc(const float* qkv, const float* E, int B, int T, int F, int axis, float* ctx, float* lse, void* stream);
 int cmgan_attention_bwd(const float* qkv, const float* E, const float* ctx, const float* dctx, const float* lse, int B, int T, int F, int axis, float* delta, float* dqkv, float* dE, void* stream);
 int cmgan_attention_bwd_tf32_parts(const float* qkv, const float* E, const float* ctx, const float* dctx, const float* lse, int B, int T, int F, int axis, float* delta, float* dqkv, float* dE, int parts, void* stream);
@@ -63,17 +69,21 @@ int cmgan_attention_bwd_tf32(const float* qkv, const float* E, const float* ctx,
 
 /* ---- GLU + depthwise conv k=31 (conformer.py:30-48,164-168) */
 int cmgan_glu_dwconv_fwd(const float* g, const float* w, const float* bias, int B, int T, int F, int axis, float* out, double* bn_sums, void* stream);
+int cmgan_glu_dwconv_fwd_varlen(const float* g, const float* w, const float* bias, int B, int T, int F, int axis, const int* frames, float* out, void* stream);
 int cmgan_glu_dwconv_bwd(const float* g, const float* dz, const float* w, int B, int T, int F, int axis, float* dg, float* dw, float* dbias, void* stream);
 
 /* ---- signal front / back end (train.py:75-112, evaluation.py:21-51, utils.py:20-39) */
 int cmgan_rms_scale(const float* x, long long ldx, int B, int L, float* c, void* stream);
 int cmgan_pad_reflect(const float* x, long long ldx, int B, int L, const float* c, float* xp, int Lp, void* stream);
+int cmgan_rms_scale_varlen(const float* x, long long ldx, int B, const int* lens, float* c, void* stream);
+int cmgan_wrap_pad_reflect_varlen(const float* x, long long ldx, int B, const int* lens, const float* c, float* xp, int Lp, void* stream);
 int cmgan_compress(const float* S, int B, int T, float* X, void* stream);
 int cmgan_uncompress(const float* re, const float* im, long long sb, long long st, long long sf, int B, int T, float* U, void* stream);
 int cmgan_uncompress_bwd(const float* re, const float* im, long long sb, long long st, long long sf, int B, int T, const float* dU, float* dre, float* dim_, int accumulate, void* stream);
 int cmgan_power_law(const float* re, const float* im, long long i0, long long i1, long long i2, float* ore, float* oim, long long o0, long long o1, long long o2, int d0, int d1, int d2, float p, void* stream);
 int cmgan_power_law_bwd(const float* re, const float* im, long long i0, long long i1, long long i2, const float* gre, const float* gim, long long o0, long long o1, long long o2, float* dre, float* dim_, long long q0, long long q1, long long q2, int d0, int d1, int d2, float p, void* stream);
 int cmgan_ola(const float* frames, int B, int T, const float* inv_env, const float* c_div, float* y, long long ldy, void* stream);
+int cmgan_ola_varlen(const float* frames, int B, int T, const int* nframes, const double* win_sq, const float* c_div, float* y, long long ldy, void* stream);
 int cmgan_ola_bwd(const float* dy, long long lddy, int B, int T, const float* inv_env, float* dframes, void* stream);
 
 /* ---- generator head and tails (generator.py:53,126,136-139,150,175-196) */
@@ -117,11 +127,14 @@ int cmgan_stoi_f64(const double* clean, const double* proc, long long L, const d
  * params = every floating-point state_dict tensor of the reference TSCNet(64, 201) in state_dict order, each starting at a multiple of 4
  * floats (cmgan_tscnet_param_info enumerates key / offset / numel; cmgan_tscnet_param_floats = size of the block).  x is (B, 2, T, F) with
  * element strides (the reference passes a permuted view, train.py:95); outputs are contiguous (B, 1, T, F).  The workspace is caller-owned,
- * 256-byte aligned, at least cmgan_tscnet_workspace_bytes(B, T, F, precision) bytes; precision 0 = exact fp32, 1 = tf32 tensor cores. */
+ * 256-byte aligned, at least cmgan_tscnet_workspace_bytes(B, T, F, precision) bytes; precision 0 = exact fp32, 1 = tf32 tensor cores.
+ * cmgan_tscnet_fwd_varlen: ragged batch of utterances padded to T frames, frames = device int[B] with 1 <= frames[b] <= T; rows t < frames[b]
+ * equal cmgan_tscnet_fwd on x[b, :, :frames[b]] alone, rows beyond are unspecified; frames == NULL is cmgan_tscnet_fwd; same workspace. */
 int cmgan_tscnet_param_count(void);
 long long cmgan_tscnet_param_floats(void);
 int cmgan_tscnet_param_info(int index, const char** key, long long* offset, long long* numel);
 long long cmgan_tscnet_workspace_bytes(int B, int T, int F, int precision);
+int cmgan_tscnet_fwd_varlen(const float* params, const float* x, long long sxb, long long sxc, long long sxt, long long sxf, int B, int T, int F, const int* frames, float* final_real, float* final_imag, void* workspace, long long workspace_bytes, int precision, void* stream);
 int cmgan_tscnet_fwd(const float* params, const float* x, long long sxb, long long sxc, long long sxt, long long sxf, int B, int T, int F, float* final_real, float* final_imag, void* workspace, long long workspace_bytes, int precision, void* stream);
 
 #ifdef __cplusplus
